@@ -2,7 +2,7 @@
 """bench.py -- one "step" = one pass of the hot path over one batch of synthetic input.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--model resnet50|bert|resnet50_int8|gpt2]
+                  [--model resnet50|bert|resnet50_int8|gpt2] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1]: the post-fusion ResNet-50 fp32 op list, batch 32 per GPU.  Prints ONE
 JSON line (rank 0).
@@ -20,6 +20,12 @@ JSON line (rank 0).
             tensor peak measured in this run (cuBLASLt 8192^3 through torch: burst = best of 10, sustained = 3 s).
   cpu_baseline / --impl reference: the CPU restatement of the reference path (oracle/; the Rust reference cannot be
             built here: no cargo) on the host cores, bounded sample.
+
+--dump-outputs DIR writes, after the timed steps of each measured mode, what the last timed step returned (the logits, or
+BERT's last hidden state; the all-gathered whole-job output at N > 1) as DIR/<output>_<mode>.npy in float32.  Inputs and
+weights come from fixed seeds, so two builds run with the same arguments can be compared output for output (to the
+rounding of the arithmetic mode: autotuned launch plans may differ from run to run).  The files stay within 64 MiB in
+all: an output larger than its share is stored as a fixed, seeded sample of its flattened elements.
 """
 from __future__ import annotations
 
@@ -45,6 +51,18 @@ MODELS = {
     "gpt2": dict(batch=8, unit="tokens/s", metric="gpt2_int8_decode_tokens_per_sec", modes=["int8"]),
 }
 GPT2_PREFILL, GPT2_CACHE = 512, 576
+OUTPUT_NAME = {"resnet50": "logits", "resnet50_int8": "logits", "bert": "last_hidden_state", "gpt2": "logits"}
+DUMP_BYTES = 64 << 20
+
+
+def dump_output(dirname, name, a, budget):
+    """DIR/<name>.npy in float32; above `budget` bytes, a fixed seeded sample of the flattened elements (ascending order)."""
+    a = np.ascontiguousarray(a, np.float32)
+    if a.nbytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, budget // a.itemsize, replace=False))
+        a = a.reshape(-1)[idx]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def load_peaks():
@@ -302,7 +320,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary numbers (other configs, 8192^3 GEMM TFLOP/s)")
     ap.add_argument("--no-peaks", action="store_true", help="skip the on-box cuBLAS peak measurement (uses MEASURED_PEAKS.json ratios)")
     ap.add_argument("--modes", default=None, help="comma list restricting the f32 modes measured (tf32,tf32x3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<output>_<mode>.npy (float32, 64 MiB at most in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     model = args.model
     batch = int(os.environ.get("RTEN_BENCH_BATCH", MODELS[model]["batch"]))  # (the override is a tuning aid: not a BASELINE config)
@@ -453,6 +475,9 @@ def main():
             return ms, launches, clocks
 
         ms, launches, clocks = timed(device_step, args.steps, args.warmup, sampler)
+        if args.dump_outputs and rank == 0:
+            last = gather_bufs[(args.steps - 1) % 2] if world > 1 else out_t
+            dump_output(args.dump_outputs, f"{OUTPUT_NAME[model]}_{mode}", last.cpu().numpy(), DUMP_BYTES // len(modes))
         res.update(value=batch * world * args.steps / (ms / 1e3), ms_per_step=ms / args.steps, gpu_launches=int(launches), clocks=clocks,
                    cuda_graph=graph is not None, flops_per_step=flops)
         if flops:
@@ -585,6 +610,9 @@ def main():
             evs.append((s, e))
         torch.cuda.synchronize()
         clocks = sampler.stop() if sampler else None
+        if args.dump_outputs and rank == 0:
+            last = gather_buf.cpu().numpy() if world > 1 else run._g_logits.numpy()
+            dump_output(args.dump_outputs, f"{OUTPUT_NAME[model]}_{res['mode']}", last, DUMP_BYTES // len(modes))
         ms = sum(s.elapsed_time(e) for s, e in evs)
         launches = ctx.launches - l0
         if world > 1:

@@ -1,5 +1,5 @@
 """Builds tests/golden/mnist.npz from the reference's own test model (rten-onnx/test-data/mnist.onnx, the export of
-tools/train-mnist.py; BASELINE configs[0]).  Run in the build container, where /root/reference exists:
+tools/train-mnist.py; BASELINE configs[0]), stored unchanged beside this script as tests/golden/mnist.onnx:
 
     python tests/golden/make_mnist_fixture.py
 
@@ -14,7 +14,7 @@ import sys
 
 import numpy as np
 
-SRC = "/root/reference/rten-onnx/test-data/mnist.onnx"
+SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "mnist.onnx")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "mnist.npz")
 
 

@@ -1,7 +1,7 @@
 """CPU-only checks of the ONNX reader (csrc/onnx_reader.cu through rten_b200_onnx_summary; no GPU, no context): the
 assertions of the reference's own decoder test (rten-onnx/src/onnx.rs:798-849) on the MNIST test model -- re-encoded from
-tests/golden/mnist.npz by tests/onnx_writer.py, and, where the reference checkout is present (the build container), on
-rten-onnx/test-data/mnist.onnx itself -- plus the encodings a file may use for the same tensor."""
+tests/golden/mnist.npz by tests/onnx_writer.py, and on the reference's file itself (rten-onnx/test-data/mnist.onnx, stored
+as tests/golden/mnist.onnx) -- plus the encodings a file may use for the same tensor."""
 import os
 
 import numpy as np
@@ -10,7 +10,7 @@ import pytest
 import onnx_writer as W
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_MNIST = "/root/reference/rten-onnx/test-data/mnist.onnx"
+REF_MNIST = os.path.join(HERE, "golden", "mnist.onnx")  # rten-onnx/test-data/mnist.onnx, unchanged
 
 
 @pytest.fixture(scope="module")
@@ -46,7 +46,6 @@ def test_decode_mnist_reencoded(summary):
     assert s["inputs"][0]["dims"] == [-1, 1, 28, 28]  # symbolic batch dimension -> -1
 
 
-@pytest.mark.skipif(not os.path.exists(REF_MNIST), reason="reference checkout not present (GPU box)")
 def test_decode_reference_mnist_file(summary):
     s = summary(open(REF_MNIST, "rb").read())
     _assert_mnist_structure(s)
