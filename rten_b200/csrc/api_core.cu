@@ -107,7 +107,7 @@ rten_status OpScope::in(const rten_tensor* t, rten_tensor* view) {
     const size_t bytes = (size_t)span * dtype_size(t->dtype);
     void* d = nullptr;
     RTB_TRY(temp_alloc(ctx, bytes ? bytes : 16, &d));
-    if (bytes) RTB_CUDA(ctx, cudaMemcpyAsync(d, t->data, bytes, cudaMemcpyHostToDevice, rtb::launch_stream(ctx)));
+    if (bytes) RTB_CUDA(ctx, cudaMemcpyAsync(d, t->data, bytes, cudaMemcpyHostToDevice, ctx->stream));
     view->data = d;
     view->device = ctx->device;
     return RTEN_OK;
@@ -182,7 +182,7 @@ rten_status OpScope::finish(rten_status st) {
     if (st == RTEN_OK) {
         for (auto& cb : copybacks) {
             if (cb.bytes) {
-                cudaError_t e = cudaMemcpyAsync(cb.host, cb.dev, cb.bytes, cudaMemcpyDeviceToHost, rtb::launch_stream(ctx));
+                cudaError_t e = cudaMemcpyAsync(cb.host, cb.dev, cb.bytes, cudaMemcpyDeviceToHost, ctx->stream);
                 if (e != cudaSuccess) st = fail_cuda(ctx, e, "cudaMemcpyAsync(D2H)");
             }
         }
@@ -314,7 +314,6 @@ void rten_b200_ctx_destroy(rten_ctx* ctx) {
         if (ctx->tune_cache.size() > ctx->tune_loaded) tune_cache_save(ctx, tf);
     if (ctx->sk_counters) cudaFree(ctx->sk_counters);
     if (ctx->attn_cnt) cudaFree(ctx->attn_cnt);
-    seq_free(ctx);
     if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
@@ -394,7 +393,7 @@ rten_status rten_b200_copy(rten_ctx* ctx, const rten_tensor* src, rten_tensor* d
         if (!bytes) return RTEN_OK;
         cudaMemcpyKind kind = src->device < 0 ? (dst->device < 0 ? cudaMemcpyHostToHost : cudaMemcpyHostToDevice)
                                               : (dst->device < 0 ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice);
-        RTB_CUDA(ctx, cudaMemcpyAsync(dst->data, src->data, bytes, kind, rtb::launch_stream(ctx)));
+        RTB_CUDA(ctx, cudaMemcpyAsync(dst->data, src->data, bytes, kind, ctx->stream));
         if ((src->device < 0 || dst->device < 0) && !ctx->capturing) RTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         return RTEN_OK;
     }
@@ -432,7 +431,7 @@ rten_status rten_b200_debug_trace(rten_ctx* ctx, int enable, int64_t* host_out_8
     }
     if (enable) {
         if (!ctx->trace) RTB_CUDA(ctx, cudaMalloc(&ctx->trace, bytes));
-        RTB_CUDA(ctx, cudaMemsetAsync(ctx->trace, 0, bytes, rtb::launch_stream(ctx)));
+        RTB_CUDA(ctx, cudaMemsetAsync(ctx->trace, 0, bytes, ctx->stream));
     } else if (ctx->trace) {
         cudaFree(ctx->trace);
         ctx->trace = nullptr;
@@ -453,7 +452,6 @@ rten_status rten_b200_graph_begin(rten_ctx* ctx) {
 rten_status rten_b200_graph_end(rten_ctx* ctx, rten_graph** out) {
     if (!ctx || !out) return RTEN_ERR_INVALID_VALUE;
     if (!ctx->capturing) return fail(ctx, RTEN_ERR_INVALID_VALUE, "no graph capture active");
-    rten_status fs = seq_flush(ctx);  // tensor-core launches still collected for a sequence kernel
     ctx->capturing = false;
     rten_graph* g = new rten_graph();
     cudaError_t e = cudaStreamEndCapture(ctx->stream, &g->graph);
@@ -463,13 +461,6 @@ rten_status rten_b200_graph_end(rten_ctx* ctx, rten_graph** out) {
         delete g;
         capture_settle(ctx, nullptr);
         return fail_cuda(ctx, e, "graph capture/instantiate");
-    }
-    if (fs != RTEN_OK) {
-        cudaGraphExecDestroy(g->exec);
-        cudaGraphDestroy(g->graph);
-        delete g;
-        capture_settle(ctx, nullptr);
-        return fs;
     }
     g->ctx = ctx;
     ctx->graphs.push_back(g);

@@ -213,7 +213,7 @@ rten_status matmul_core(OpScope& sc, MatMulArgs& A, rten_tensor* out) {
             dv.data = t;
             copy_out = true;
         }
-        RTB_CUDA(ctx, cudaMemsetAsync(dv.data, 0, (size_t)total * 4, rtb::launch_stream(ctx)));
+        RTB_CUDA(ctx, cudaMemsetAsync(dv.data, 0, (size_t)total * 4, ctx->stream));
         if (A.kind == 0 && L.epi.bias) {
             long long shp[2] = {total / N, N}, s0[2] = {N, 1}, sb[2] = {0, 1};
             RTB_TRY(launch_nd_add(ctx, (const float*)dv.data, L.epi.bias, (float*)dv.data, 2, shp, s0, sb, s0, 0));
@@ -440,7 +440,7 @@ rten_status rten_b200_prepack_b(rten_ctx* ctx, const rten_tensor* b, rten_packed
         p->ld = round_up(std::max<int64_t>(p->K, 1), 16 / es);
         st = pool_alloc(ctx, (size_t)std::max<int64_t>(p->N * p->ld, 1) * es, &p->data);
         if (st == RTEN_OK) {
-            RTB_CUDA(ctx, cudaMemsetAsync(p->data, 0, (size_t)std::max<int64_t>(p->N * p->ld, 1) * es, rtb::launch_stream(ctx)));
+            RTB_CUDA(ctx, cudaMemsetAsync(p->data, 0, (size_t)std::max<int64_t>(p->N * p->ld, 1) * es, ctx->stream));
             long long shape[2] = {p->N, p->K}, ss[2] = {bv.strides[1], bv.strides[0]}, ds[2] = {p->ld, 1};
             st = launch_nd_copy(ctx, es, bv.data, p->data, 2, shape, ss, ds);
         }

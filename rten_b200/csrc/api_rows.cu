@@ -372,8 +372,8 @@ rten_status rten_b200_dynamic_quantize_linear_ranged(rten_ctx* ctx, const rten_t
         if (n == 0) {
             // quantize.rs:378-386: scale 1, zero point 0
             const float one = 1.0f;
-            RTB_CUDA(ctx, cudaMemcpyAsync(sv.data, &one, 4, cudaMemcpyHostToDevice, rtb::launch_stream(ctx)));
-            RTB_CUDA(ctx, cudaMemsetAsync(zv.data, 0, 1, rtb::launch_stream(ctx)));
+            RTB_CUDA(ctx, cudaMemcpyAsync(sv.data, &one, 4, cudaMemcpyHostToDevice, ctx->stream));
+            RTB_CUDA(ctx, cudaMemsetAsync(zv.data, 0, 1, ctx->stream));
         } else if (!nccl_comm && !range && !rows_out && n <= 16384) {
             st = launch_dql_small(ctx, (const float*)xc.data, (uint8_t*)yv.data, (int)n, (float*)sv.data, (uint8_t*)zv.data);
         } else {

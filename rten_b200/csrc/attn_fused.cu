@@ -296,12 +296,9 @@ rten_status launch_attn_fused(rten_ctx* ctx, const AttnFusedLaunch& L) {
     cfg.gridDim = dim3(L.B * L.heads * p.q_tiles);
     cfg.blockDim = dim3(AF_THREADS);
     cfg.dynamicSmemBytes = smem;
-    cfg.stream = launch_stream(ctx);
+    cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+    fill_launch_attrs(cfg, attr, false);
     cudaError_t e = cudaFuncSetAttribute(attn_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) e = cudaLaunchKernelEx(&cfg, attn_fused_kernel, mq, mk, mv, p);
     if (e != cudaSuccess) return fail_cuda(ctx, e, "fused attention launch");

@@ -84,7 +84,7 @@ namespace rtb {
 // min / max on that encoding is the float min / max, and is exact and order independent.
 rten_status comm_allreduce_minmax(rten_ctx* ctx, rten_comm* comm, int* mm) {
     if (!comm || comm->world <= 1) return RTEN_OK;
-    cudaStream_t s = launch_stream(ctx);
+    cudaStream_t s = ctx->stream;
     if (comm->peer_ok) {
         cudaLaunchConfig_t cfg;
         memset(&cfg, 0, sizeof(cfg));
@@ -92,10 +92,7 @@ rten_status comm_allreduce_minmax(rten_ctx* ctx, rten_comm* comm, int* mm) {
         cfg.blockDim = dim3(32);
         cfg.stream = s;
         cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+        fill_launch_attrs(cfg, attr, false);
         cudaError_t e = cudaLaunchKernelEx(&cfg, peer_minmax_kernel, mm, comm->peers, comm->rank, comm->world);
         if (e != cudaSuccess) return fail_cuda(ctx, e, "peer min/max exchange launch");
         count_launch(ctx);

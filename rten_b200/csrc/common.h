@@ -7,6 +7,7 @@
 #include <array>
 #include <cstdint>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <string>
@@ -70,9 +71,6 @@ struct rten_ctx {
     void* encode_tiled = nullptr;  // cuTensorMapEncodeTiled (driver entry point)
     void* sk_counters = nullptr;   // split-K arrival counters (zero between launches)
     bool autotune = false;         // time candidate launch plans on first sight of a problem (umma_gemm.cu)
-    void* seq_pending = nullptr;   // umma_gemm launches collected during graph capture (std::vector<PendingLaunch>*)
-    int seq_class = -1;            // kernel class (data kind, epilogue variant) of the pending launches
-    void* seq_gbar = nullptr;      // grid-barrier arrival counter of the sequence kernel
     std::map<std::vector<long long>, std::array<int, 8>> tune_cache;
     size_t tune_loaded = 0;        // entries read from RTEN_B200_TUNE_FILE (the file is rewritten when more exist at destroy)
     std::vector<rten_graph*> graphs;  // graphs captured on this context that still exist
@@ -149,13 +147,24 @@ rten_status comm_allreduce_minmax(rten_ctx* ctx, struct ::rten_comm* comm, int* 
 struct RangeExchange;
 bool comm_range_exchange(struct ::rten_comm* comm, RangeExchange* out);  // true: the quantise kernel exchanges the range itself
 
-// Deferred tensor-core launches (graph capture batches them into sequence kernels, umma_gemm.cu) must be issued
-// before anything else is enqueued on the context stream: every other launch site asks for the stream through this.
-rten_status seq_flush(rten_ctx* ctx);
-void seq_free(rten_ctx* ctx);
-inline cudaStream_t launch_stream(rten_ctx* ctx) {
-    if (ctx->seq_pending) seq_flush(ctx);
-    return ctx->stream;
+// Launch attributes of a cudaLaunchKernelEx launch: programmatic dependent launch (unless RTEN_B200_NO_PDL is set, read
+// at every launch) and, with `cluster2`, a 2x1x1 cluster.  `attr` must hold two entries when `cluster2` is set.
+inline void fill_launch_attrs(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr, bool cluster2) {
+    int nattr = 0;
+    if (!getenv("RTEN_B200_NO_PDL")) {
+        attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[nattr].val.programmaticStreamSerializationAllowed = 1;
+        nattr++;
+    }
+    if (cluster2) {
+        attr[nattr].id = cudaLaunchAttributeClusterDimension;
+        attr[nattr].val.clusterDim.x = 2;
+        attr[nattr].val.clusterDim.y = 1;
+        attr[nattr].val.clusterDim.z = 1;
+        nattr++;
+    }
+    cfg.attrs = attr;
+    cfg.numAttrs = nattr;
 }
 
 }  // namespace rtb

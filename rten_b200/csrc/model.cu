@@ -134,7 +134,7 @@ rten_status upload_constant(rten_model* m, const onnx::Tensor& t, ValueSlot* v) 
     void* d = nullptr;
     RTB_TRY(pool_alloc(ctx, bytes ? bytes : 16, &d));
     m->const_allocs.push_back(d);
-    if (bytes) RTB_CUDA(ctx, cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, launch_stream(ctx)));
+    if (bytes) RTB_CUDA(ctx, cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
     RTB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // `conv` / the file buffer may go away
     v->kind = V_CONST;
     v->t.data = d;

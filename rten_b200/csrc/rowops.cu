@@ -271,7 +271,7 @@ rten_status launch_softmax(rten_ctx* ctx, const float* x, float* y, long long ro
         const unsigned blocks = (unsigned)((warps + vwpb - 1) / vwpb);
         const int F = n / (16 * S);
         const int fm = F <= 2 ? 2 : (F <= 4 ? 4 : (F <= 8 ? 8 : 16));
-        cudaStream_t st = launch_stream(ctx);
+        cudaStream_t st = ctx->stream;
 #define RTB_SOFTMAX_CASE(SS, FF) \
     case SS * 100 + FF: softmax_vec_kernel<SS, FF><<<blocks, vwpb * 32, 0, st>>>(p); break;
         switch (S * 100 + fm) {
@@ -287,7 +287,7 @@ rten_status launch_softmax(rten_ctx* ctx, const float* x, float* y, long long ro
         return RTEN_OK;
     }
     const long long blocks = (rows + wpb - 1) / wpb;
-    softmax_kernel<<<(unsigned)blocks, wpb * 32, 0, launch_stream(ctx)>>>(p);
+    softmax_kernel<<<(unsigned)blocks, wpb * 32, 0, ctx->stream>>>(p);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "softmax launch");
     count_launch(ctx);
@@ -447,7 +447,7 @@ rten_status launch_layer_norm(rten_ctx* ctx, const float* x, float* y, long long
         const unsigned blocks = (unsigned)((warps + vwpb - 1) / vwpb);
         const int F = n / (64 * S);
         const int fm = F <= 4 ? 4 : (F <= 8 ? 8 : (F <= 12 ? 12 : 16));
-        cudaStream_t st = launch_stream(ctx);
+        cudaStream_t st = ctx->stream;
 #define RTB_LN_CASE(SS, FF) \
     case SS * 100 + FF: layer_norm_vec_kernel<SS, FF><<<blocks, vwpb * 32, 0, st>>>(p); break;
         switch (S * 100 + fm) {
@@ -457,7 +457,7 @@ rten_status launch_layer_norm(rten_ctx* ctx, const float* x, float* y, long long
 #undef RTB_LN_CASE
     } else {
         const long long blocks = (rows + wpb - 1) / wpb;
-        layer_norm_kernel<<<(unsigned)blocks, wpb * 32, 0, launch_stream(ctx)>>>(p);
+        layer_norm_kernel<<<(unsigned)blocks, wpb * 32, 0, ctx->stream>>>(p);
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "layer_norm launch");
@@ -533,7 +533,7 @@ rten_status launch_row_mean(rten_ctx* ctx, const float* x, float* y, long long r
                             long long s_outer, long long s_inner, long long kstride) {
     if (rows == 0) return RTEN_OK;
     if (s_inner == 1 && kstride != 1) {
-        row_mean_thread_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, launch_stream(ctx)>>>(x, y, rows, n, rows_inner, s_outer,
+        row_mean_thread_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, ctx->stream>>>(x, y, rows, n, rows_inner, s_outer,
                                                                                         s_inner, kstride);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return fail_cuda(ctx, e, "row_mean launch");
@@ -541,7 +541,7 @@ rten_status launch_row_mean(rten_ctx* ctx, const float* x, float* y, long long r
         return RTEN_OK;
     }
     const int wpb = 8;
-    row_mean_kernel<<<(unsigned)((rows + wpb - 1) / wpb), wpb * 32, 0, launch_stream(ctx)>>>(x, y, rows, n, rows_inner,
+    row_mean_kernel<<<(unsigned)((rows + wpb - 1) / wpb), wpb * 32, 0, ctx->stream>>>(x, y, rows, n, rows_inner,
                                                                                        s_outer, s_inner, kstride);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "row_mean launch");
@@ -593,10 +593,10 @@ rten_status launch_unary(rten_ctx* ctx, int op, const float* x, float* y, long l
     const int vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0 ? 1 : 0;
     const int grid = ew_grid(ctx, vec ? (n + 3) / 4 : n);
     switch (op) {
-        case UNARY_ERF: unary_kernel<UNARY_ERF><<<grid, 256, 0, launch_stream(ctx)>>>(x, y, n, vec); break;
-        case UNARY_GELU: unary_kernel<UNARY_GELU><<<grid, 256, 0, launch_stream(ctx)>>>(x, y, n, vec); break;
-        case UNARY_APPROX_GELU: unary_kernel<UNARY_APPROX_GELU><<<grid, 256, 0, launch_stream(ctx)>>>(x, y, n, vec); break;
-        case UNARY_RELU: unary_kernel<UNARY_RELU><<<grid, 256, 0, launch_stream(ctx)>>>(x, y, n, vec); break;
+        case UNARY_ERF: unary_kernel<UNARY_ERF><<<grid, 256, 0, ctx->stream>>>(x, y, n, vec); break;
+        case UNARY_GELU: unary_kernel<UNARY_GELU><<<grid, 256, 0, ctx->stream>>>(x, y, n, vec); break;
+        case UNARY_APPROX_GELU: unary_kernel<UNARY_APPROX_GELU><<<grid, 256, 0, ctx->stream>>>(x, y, n, vec); break;
+        case UNARY_RELU: unary_kernel<UNARY_RELU><<<grid, 256, 0, ctx->stream>>>(x, y, n, vec); break;
         default: return fail(ctx, RTEN_ERR_INVALID_VALUE, "unknown unary op");
     }
     cudaError_t e = cudaGetLastError();
@@ -730,11 +730,11 @@ rten_status launch_nd_copy(rten_ctx* ctx, int esize, const void* src, void* dst,
     }
     const int grid = ew_grid(ctx, p.n);
     switch (es) {
-        case 1: nd_copy_kernel<uint8_t><<<grid, 256, 0, launch_stream(ctx)>>>((const uint8_t*)src, (uint8_t*)dst, p); break;
-        case 2: nd_copy_kernel<uint16_t><<<grid, 256, 0, launch_stream(ctx)>>>((const uint16_t*)src, (uint16_t*)dst, p); break;
-        case 4: nd_copy_kernel<uint32_t><<<grid, 256, 0, launch_stream(ctx)>>>((const uint32_t*)src, (uint32_t*)dst, p); break;
-        case 8: nd_copy_kernel<uint2><<<grid, 256, 0, launch_stream(ctx)>>>((const uint2*)src, (uint2*)dst, p); break;
-        default: nd_copy_kernel<uint4><<<grid, 256, 0, launch_stream(ctx)>>>((const uint4*)src, (uint4*)dst, p); break;
+        case 1: nd_copy_kernel<uint8_t><<<grid, 256, 0, ctx->stream>>>((const uint8_t*)src, (uint8_t*)dst, p); break;
+        case 2: nd_copy_kernel<uint16_t><<<grid, 256, 0, ctx->stream>>>((const uint16_t*)src, (uint16_t*)dst, p); break;
+        case 4: nd_copy_kernel<uint32_t><<<grid, 256, 0, ctx->stream>>>((const uint32_t*)src, (uint32_t*)dst, p); break;
+        case 8: nd_copy_kernel<uint2><<<grid, 256, 0, ctx->stream>>>((const uint2*)src, (uint2*)dst, p); break;
+        default: nd_copy_kernel<uint4><<<grid, 256, 0, ctx->stream>>>((const uint4*)src, (uint4*)dst, p); break;
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "nd_copy launch");
@@ -784,7 +784,7 @@ rten_status launch_nd_add(rten_ctx* ctx, const float* a, const float* b, float* 
         }
         if (ok && in_bcast && period > 0 && (period & 3) == 0 && n < 0x7fffffffLL && n > 0 &&
             ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(d)) & 15) == 0) {
-            add_periodic_kernel<<<ew_grid(ctx, n / 4), 256, 0, launch_stream(ctx)>>>(reinterpret_cast<const float4*>(a), reinterpret_cast<const float4*>(b),
+            add_periodic_kernel<<<ew_grid(ctx, n / 4), 256, 0, ctx->stream>>>(reinterpret_cast<const float4*>(a), reinterpret_cast<const float4*>(b),
                                                                                reinterpret_cast<float4*>(d), (unsigned)(n / 4), (unsigned)(period / 4), relu);
             cudaError_t e = cudaGetLastError();
             if (e != cudaSuccess) return fail_cuda(ctx, e, "nd_add launch");
@@ -804,7 +804,7 @@ rten_status launch_nd_add(rten_ctx* ctx, const float* a, const float* b, float* 
         p.n *= shape[i];
     }
     if (p.n == 0) return RTEN_OK;
-    nd_add_kernel<<<ew_grid(ctx, p.n), 256, 0, launch_stream(ctx)>>>(a, b, d, p, relu);
+    nd_add_kernel<<<ew_grid(ctx, p.n), 256, 0, ctx->stream>>>(a, b, d, p, relu);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "nd_add launch");
     count_launch(ctx);
@@ -819,7 +819,7 @@ rten_status launch_add_flat(rten_ctx* ctx, const float* a, const float* b, float
         long long shape[1] = {n}, s1[1] = {1};
         return launch_nd_add(ctx, a, b, d, 1, shape, s1, s1, s1, relu);
     }
-    add_flat_kernel<<<ew_grid(ctx, (n + 3) / 4), 256, 0, launch_stream(ctx)>>>(a, b, d, n, relu);
+    add_flat_kernel<<<ew_grid(ctx, (n + 3) / 4), 256, 0, ctx->stream>>>(a, b, d, n, relu);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "add launch");
     count_launch(ctx);
@@ -993,7 +993,7 @@ rten_status launch_dql_quantize_rows(rten_ctx* ctx, const float* x, uint8_t* y, 
     if (total == 0) return RTEN_OK;
     RangeExchange none;
     memset(&none, 0, sizeof(none));
-    dql_quantize_rows_kernel<<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>(x, y, rows, row_len, rows_inner, y_inner, y_outer,
+    dql_quantize_rows_kernel<<<ew_grid(ctx, total), 256, 0, ctx->stream>>>(x, y, rows, row_len, rows_inner, y_inner, y_outer,
                                                                           mm, scale_out, zp_out, xch ? *xch : none);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "dql launch");
@@ -1002,7 +1002,7 @@ rten_status launch_dql_quantize_rows(rten_ctx* ctx, const float* x, uint8_t* y, 
 }
 
 rten_status launch_dql_small(rten_ctx* ctx, const float* x, uint8_t* y, int n, float* scale_out, uint8_t* zp_out) {
-    dql_small_kernel<<<1, 1024, 0, launch_stream(ctx)>>>(x, y, n, scale_out, zp_out);
+    dql_small_kernel<<<1, 1024, 0, ctx->stream>>>(x, y, n, scale_out, zp_out);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "dql launch");
     count_launch(ctx);
@@ -1019,7 +1019,7 @@ __global__ void range_reset_kernel(int* mm, int pairs) {
 
 rten_status launch_range_reset(rten_ctx* ctx, int* mm, int pairs) {
     if (pairs == 0) return RTEN_OK;
-    range_reset_kernel<<<(pairs + 127) / 128, 128, 0, launch_stream(ctx)>>>(mm, pairs);
+    range_reset_kernel<<<(pairs + 127) / 128, 128, 0, ctx->stream>>>(mm, pairs);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "range reset launch");
     count_launch(ctx);
@@ -1027,10 +1027,10 @@ rten_status launch_range_reset(rten_ctx* ctx, int* mm, int pairs) {
 }
 
 rten_status launch_minmax(rten_ctx* ctx, const float* x, long long n, int* mm) {
-    minmax_init_kernel<<<1, 1, 0, launch_stream(ctx)>>>(mm);
+    minmax_init_kernel<<<1, 1, 0, ctx->stream>>>(mm);
     count_launch(ctx);
     if (n > 0) {
-        minmax_kernel<<<ew_grid(ctx, (n + 3) / 4), 256, 0, launch_stream(ctx)>>>(x, n, mm);
+        minmax_kernel<<<ew_grid(ctx, (n + 3) / 4), 256, 0, ctx->stream>>>(x, n, mm);
         count_launch(ctx);
     }
     cudaError_t e = cudaGetLastError();
@@ -1042,7 +1042,7 @@ rten_status launch_dql_quantize(rten_ctx* ctx, const float* x, uint8_t* y, long 
                                 uint8_t* zp_out, const RangeExchange* xch) {
     RangeExchange none;
     memset(&none, 0, sizeof(none));
-    dql_quantize_kernel<<<ew_grid(ctx, (n + 15) / 16), 256, 0, launch_stream(ctx)>>>(x, y, n, mm, scale_out, zp_out, xch ? *xch : none);
+    dql_quantize_kernel<<<ew_grid(ctx, (n + 15) / 16), 256, 0, ctx->stream>>>(x, y, n, mm, scale_out, zp_out, xch ? *xch : none);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "dql launch");
     count_launch(ctx);
@@ -1069,7 +1069,7 @@ rowsum8_kernel(const uint8_t* __restrict__ a, int is_signed, long long rows, int
 rten_status launch_rowsum8(rten_ctx* ctx, const void* a, int is_signed, long long rows, int K, long long ld, int* out) {
     if (rows == 0) return RTEN_OK;
     const int wpb = 8;
-    rowsum8_kernel<<<(unsigned)((rows + wpb - 1) / wpb), wpb * 32, 0, launch_stream(ctx)>>>((const uint8_t*)a, is_signed, rows,
+    rowsum8_kernel<<<(unsigned)((rows + wpb - 1) / wpb), wpb * 32, 0, ctx->stream>>>((const uint8_t*)a, is_signed, rows,
                                                                                       K, ld, out);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "rowsum launch");
@@ -1085,7 +1085,7 @@ __global__ void zp_to_i32_kernel(const uint8_t* zp, int is_signed, int n, long l
 
 rten_status launch_zp_to_i32(rten_ctx* ctx, const void* zp, int is_signed, int n, long long zs, int* out) {
     if (n == 0) return RTEN_OK;
-    zp_to_i32_kernel<<<(n + 127) / 128, 128, 0, launch_stream(ctx)>>>((const uint8_t*)zp, is_signed, n, zs, out);
+    zp_to_i32_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>((const uint8_t*)zp, is_signed, n, zs, out);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "zp_to_i32 launch");
     count_launch(ctx);
@@ -1098,7 +1098,7 @@ __global__ void fill8_kernel(uint8_t* p, long long n, uint8_t v) {
 }
 rten_status launch_fill8(rten_ctx* ctx, void* p, long long n, uint8_t v) {
     if (n == 0) return RTEN_OK;
-    fill8_kernel<<<ew_grid(ctx, n), 256, 0, launch_stream(ctx)>>>((uint8_t*)p, n, v);
+    fill8_kernel<<<ew_grid(ctx, n), 256, 0, ctx->stream>>>((uint8_t*)p, n, v);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "fill launch");
     count_launch(ctx);
@@ -1116,7 +1116,7 @@ cast_scale_kernel(const int* __restrict__ in, float* __restrict__ out, long long
 rten_status launch_cast_scale(rten_ctx* ctx, const int* in, float* out, long long n, int cols, const float* scale,
                               int scale_len) {
     if (n == 0) return RTEN_OK;
-    cast_scale_kernel<<<ew_grid(ctx, n), 256, 0, launch_stream(ctx)>>>(in, out, n, cols, scale, scale_len);
+    cast_scale_kernel<<<ew_grid(ctx, n), 256, 0, ctx->stream>>>(in, out, n, cols, scale, scale_len);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "cast_scale launch");
     count_launch(ctx);
@@ -1179,9 +1179,9 @@ rten_status launch_im2col(rten_ctx* ctx, int esize, const void* x, void* out, co
     if (total == 0) return RTEN_OK;
     if (esize == 4) {
         float pv = 0.0f;
-        im2col_kernel<float><<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>((const float*)x, (float*)out, p, pv);
+        im2col_kernel<float><<<ew_grid(ctx, total), 256, 0, ctx->stream>>>((const float*)x, (float*)out, p, pv);
     } else {
-        im2col_kernel<uint8_t><<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>((const uint8_t*)x, (uint8_t*)out, p,
+        im2col_kernel<uint8_t><<<ew_grid(ctx, total), 256, 0, ctx->stream>>>((const uint8_t*)x, (uint8_t*)out, p,
                                                                              (uint8_t)pad_value);
     }
     cudaError_t e = cudaGetLastError();
@@ -1232,7 +1232,7 @@ rten_status launch_smallc_pad(rten_ctx* ctx, const float* x, float* xp, int B, i
                               long long xs_b, long long xs_c, long long xs_h, long long xs_w) {
     const long long total = (long long)B * H * Wp;
     if (total == 0) return RTEN_OK;
-    smallc_pad_kernel<<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>(x, xp, B, C, H, W, Wp, pl, xs_b, xs_c, xs_h, xs_w);
+    smallc_pad_kernel<<<ew_grid(ctx, total), 256, 0, ctx->stream>>>(x, xp, B, C, H, W, Wp, pl, xs_b, xs_c, xs_h, xs_w);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "smallc_pad launch");
     count_launch(ctx);
@@ -1243,7 +1243,7 @@ rten_status launch_smallc_pack_w(rten_ctx* ctx, const float* w, float* wp, int O
                                  long long ws_c, long long ws_h, long long ws_w) {
     const int total = O * kh * 32;
     if (total == 0) return RTEN_OK;
-    smallc_pack_w_kernel<<<(total + 255) / 256, 256, 0, launch_stream(ctx)>>>(w, wp, O, C, kh, kw, ws_o, ws_c, ws_h, ws_w);
+    smallc_pack_w_kernel<<<(total + 255) / 256, 256, 0, ctx->stream>>>(w, wp, O, C, kh, kw, ws_o, ws_c, ws_h, ws_w);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "smallc_pack_w launch");
     count_launch(ctx);
@@ -1328,9 +1328,9 @@ rten_status launch_maxpool(rten_ctx* ctx, const float* x, float* y, const PoolPa
                      (p.xs_w % 4) == 0 && (p.ys_b % 4) == 0 && (p.ys_h % 4) == 0 && (p.ys_w % 4) == 0 &&
                      ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0;
     if (cl4)
-        maxpool_cl4_kernel<<<ew_grid(ctx, total / 4), 256, 0, launch_stream(ctx)>>>(x, y, p);
+        maxpool_cl4_kernel<<<ew_grid(ctx, total / 4), 256, 0, ctx->stream>>>(x, y, p);
     else
-        maxpool_kernel<<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>(x, y, p);
+        maxpool_kernel<<<ew_grid(ctx, total), 256, 0, ctx->stream>>>(x, y, p);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "maxpool launch");
     count_launch(ctx);
@@ -1369,14 +1369,14 @@ rten_status launch_gather_rows(rten_ctx* ctx, const float* table, const int* idx
     if (nidx * width == 0) return RTEN_OK;
     if (t_cs == 1 && (width & 3) == 0 && (t_rs & 3) == 0 && nidx * width < 0x7fffffffLL &&
         ((reinterpret_cast<uintptr_t>(table) | reinterpret_cast<uintptr_t>(out)) & 15) == 0) {
-        gather_rows_vec_kernel<<<ew_grid(ctx, nidx * width / 4), 256, 0, launch_stream(ctx)>>>(table, idx, reinterpret_cast<float4*>(out),
+        gather_rows_vec_kernel<<<ew_grid(ctx, nidx * width / 4), 256, 0, ctx->stream>>>(table, idx, reinterpret_cast<float4*>(out),
                                                                                        (unsigned)(nidx * width / 4), (unsigned)(width / 4), t_rs, rows);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return fail_cuda(ctx, e, "gather launch");
         count_launch(ctx);
         return RTEN_OK;
     }
-    gather_rows_kernel<<<ew_grid(ctx, nidx * width), 256, 0, launch_stream(ctx)>>>(table, idx, out, nidx, width, t_rs, t_cs,
+    gather_rows_kernel<<<ew_grid(ctx, nidx * width), 256, 0, ctx->stream>>>(table, idx, out, nidx, width, t_rs, t_cs,
                                                                             rows);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "gather launch");
@@ -1430,7 +1430,7 @@ rten_status launch_smallc8_pad(rten_ctx* ctx, const void* x, void* xp, int B, in
                                int pl, long long xs_b, long long xs_c, long long xs_h, long long xs_w, int pad_value) {
     const long long total = (long long)B * Hp * Wp;
     if (total == 0) return RTEN_OK;
-    smallc8_pad_kernel<<<ew_grid(ctx, total), 256, 0, launch_stream(ctx)>>>((const uint8_t*)x, (uint8_t*)xp, B, C, H, W, Hp, Wp,
+    smallc8_pad_kernel<<<ew_grid(ctx, total), 256, 0, ctx->stream>>>((const uint8_t*)x, (uint8_t*)xp, B, C, H, W, Hp, Wp,
                                                                      pt, pl, xs_b, xs_c, xs_h, xs_w, pad_value);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "smallc8 pad launch");
@@ -1442,7 +1442,7 @@ rten_status launch_smallc8_pack_w(rten_ctx* ctx, const void* w, void* wp, int O,
                                   long long ws_c, long long ws_h, long long ws_w) {
     const int total = O * kh * 128;
     if (total == 0) return RTEN_OK;
-    smallc8_pack_w_kernel<<<(total + 255) / 256, 256, 0, launch_stream(ctx)>>>((const uint8_t*)w, (uint8_t*)wp, O, C, kh, kw,
+    smallc8_pack_w_kernel<<<(total + 255) / 256, 256, 0, ctx->stream>>>((const uint8_t*)w, (uint8_t*)wp, O, C, kh, kw,
                                                                          ws_o, ws_c, ws_h, ws_w);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "smallc8 pack launch");
@@ -1469,7 +1469,7 @@ scatter_rows_kernel(float* __restrict__ table, const int* __restrict__ idx, cons
 rten_status launch_scatter_rows(rten_ctx* ctx, float* table, const int* idx, const float* src, long long nidx, int width,
                                 long long t_rs, long long t_cs, long long s_rs, long long s_cs, long long rows) {
     if (nidx * width == 0) return RTEN_OK;
-    scatter_rows_kernel<<<ew_grid(ctx, nidx * width), 256, 0, launch_stream(ctx)>>>(table, idx, src, nidx, width, t_rs, t_cs,
+    scatter_rows_kernel<<<ew_grid(ctx, nidx * width), 256, 0, ctx->stream>>>(table, idx, src, nidx, width, t_rs, t_cs,
                                                                              s_rs, s_cs, rows);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "scatter launch");
@@ -1590,7 +1590,7 @@ rten_status launch_tf32x3_split(rten_ctx* ctx, const float* x, float* y, const l
                        (p.d3 == 1 || p.s3 == p.d0 * p.d1 * p.d2) && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
                        (reinterpret_cast<uintptr_t>(y) & 15) == 0;
     if (dense) {
-        tf32x3_lo_flat_kernel<<<ew_grid(ctx, p.n / 16), 256, 0, launch_stream(ctx)>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<float4*>(y), p.n / 4);
+        tf32x3_lo_flat_kernel<<<ew_grid(ctx, p.n / 16), 256, 0, ctx->stream>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<float4*>(y), p.n / 4);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return fail_cuda(ctx, e, "tf32x3 split launch");
         count_launch(ctx);
@@ -1599,9 +1599,9 @@ rten_status launch_tf32x3_split(rten_ctx* ctx, const float* x, float* y, const l
     const bool vec = (p.d0 & 3) == 0 && (p.d0p & 3) == 0 && (p.s1 & 3) == 0 && (p.s2 & 3) == 0 && (p.s3 & 3) == 0 &&
                      (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0 && p.n < 0x7fffffffLL;
     if (vec)
-        tf32x3_split_vec_kernel<<<ew_grid(ctx, p.n / 4), 256, 0, launch_stream(ctx)>>>(x, y, p);
+        tf32x3_split_vec_kernel<<<ew_grid(ctx, p.n / 4), 256, 0, ctx->stream>>>(x, y, p);
     else
-        tf32x3_split_kernel<<<ew_grid(ctx, p.n), 256, 0, launch_stream(ctx)>>>(x, y, p);
+        tf32x3_split_kernel<<<ew_grid(ctx, p.n), 256, 0, ctx->stream>>>(x, y, p);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail_cuda(ctx, e, "tf32x3 split launch");
     count_launch(ctx);

@@ -406,12 +406,9 @@ rten_status launch_qlinear(rten_ctx* ctx, const QLinearLaunch& L) {
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(256);
     cfg.dynamicSmemBytes = smem;
-    cfg.stream = launch_stream(ctx);
+    cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+    fill_launch_attrs(cfg, attr, false);
     auto go = [&](auto kern) -> cudaError_t {
         if (smem > 48 * 1024) {
             cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -548,12 +545,9 @@ rten_status launch_skinny_f32(rten_ctx* ctx, const SkinnyF32Launch& L) {
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(256);
     cfg.dynamicSmemBytes = smem;
-    cfg.stream = launch_stream(ctx);
+    cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+    fill_launch_attrs(cfg, attr, false);
     auto go = [&](auto kern) -> cudaError_t {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
         if (e != cudaSuccess) return e;
@@ -867,12 +861,9 @@ rten_status launch_attn_decode(rten_ctx* ctx, const AttnDecodeLaunch& L) {
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(bh * ns);
     cfg.blockDim = dim3(nw * 32);
-    cfg.stream = launch_stream(ctx);
+    cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+    fill_launch_attrs(cfg, attr, false);
     cudaError_t e = L.dh == 64 ? (nw == 6 ? cudaLaunchKernelEx(&cfg, attn_decode_kernel<64, 6>, p) : cudaLaunchKernelEx(&cfg, attn_decode_kernel<64, 8>, p))
                                : cudaLaunchKernelEx(&cfg, attn_decode_kernel<128, 8>, p);
     if (e != cudaSuccess) return fail_cuda(ctx, e, "attention launch");

@@ -263,7 +263,7 @@ __device__ __forceinline__ void epilogue_fast(const EpiCtx& c) {
     }
     if (e.range) range_commit(e.range, rg_lo, rg_hi);
     // shared memory must stay valid until the last bulk store has READ it; the global writes complete on their own
-    // before the grid is considered finished (a sequence kernel waits for them at its layer boundary)
+    // before the grid is considered finished
     if (issuer) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 

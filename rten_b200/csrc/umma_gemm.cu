@@ -30,7 +30,6 @@
 #include <algorithm>
 #include <array>
 #include <cmath>
-#include <memory>
 #include <vector>
 #include <cmath>
 #include <cstdint>
@@ -388,45 +387,15 @@ static rten_status ensure_splitk_counters(rten_ctx* ctx) {
     return RTEN_OK;
 }
 
-struct PendingLaunch {
+struct LaunchArgs {
     bool plain = false;  // f32 launch that qualifies for the plain epilogue (kernel variant 3; a subset of variant 1)
     KParams p;
     CUtensorMap maps[5];  // a, b, d, residual, a2 (two-plane 3xTF32: low parts of A)
     size_t smem_bytes;
 };
 
-static std::vector<PendingLaunch>* pending_of(rten_ctx* ctx) {
-    if (!ctx->seq_pending) ctx->seq_pending = new std::vector<PendingLaunch>();
-    return reinterpret_cast<std::vector<PendingLaunch>*>(ctx->seq_pending);
-}
-
-void seq_free(rten_ctx* ctx) {
-    if (ctx->seq_pending) delete reinterpret_cast<std::vector<PendingLaunch>*>(ctx->seq_pending);
-    ctx->seq_pending = nullptr;
-    if (ctx->seq_gbar) cudaFree(ctx->seq_gbar);
-    ctx->seq_gbar = nullptr;
-}
-
-static void fill_launch_attrs(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr, bool cluster2) {
-    int nattr = 0;
-    if (!getenv("RTEN_B200_NO_PDL")) {
-        attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-        nattr++;
-    }
-    if (cluster2) {
-        attr[nattr].id = cudaLaunchAttributeClusterDimension;
-        attr[nattr].val.clusterDim.x = 2;
-        attr[nattr].val.clusterDim.y = 1;
-        attr[nattr].val.clusterDim.z = 1;
-        nattr++;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = nattr;
-}
-
 // cls = kind * 3 + epilogue variant
-static rten_status launch_single(rten_ctx* ctx, int cls, const PendingLaunch& pl) {
+static rten_status launch_single(rten_ctx* ctx, int cls, const LaunchArgs& pl) {
     const KParams& p = pl.p;
     const int grid = p.cta2 ? 2 * std::min(p.units_total, ctx->num_sms / 2) : std::min(p.units_total, ctx->num_sms);
     cudaLaunchConfig_t cfg;
@@ -473,62 +442,8 @@ static rten_status launch_single(rten_ctx* ctx, int cls, const PendingLaunch& pl
     return RTEN_OK;
 }
 
-// Launch whatever umma_gemm launches are pending on this context (one: the plain kernel; several: the sequence kernel).
-rten_status seq_flush(rten_ctx* ctx) {
-    if (!ctx->seq_pending) return RTEN_OK;
-    auto* q = reinterpret_cast<std::vector<PendingLaunch>*>(ctx->seq_pending);
-    if (q->empty()) return RTEN_OK;
-    std::vector<PendingLaunch> items;
-    items.swap(*q);  // (re-entrancy: launch paths below call seq_flush through launch_stream)
-    const int cls = ctx->seq_class;
-    if (items.size() == 1) return launch_single(ctx, cls, items[0]);
-    if (!ctx->seq_gbar) {
-        cudaError_t ce = cudaMalloc(&ctx->seq_gbar, 256);
-        if (ce != cudaSuccess) return fail_cuda(ctx, ce, "sequence barrier");
-        ce = cudaMemset(ctx->seq_gbar, 0, 256);
-        if (ce != cudaSuccess) return fail_cuda(ctx, ce, "sequence barrier");
-    }
-    std::unique_ptr<SeqParams> sp(new SeqParams());
-    memset(sp.get(), 0, sizeof(SeqParams));
-    sp->n = (int)items.size();
-    sp->gbar = reinterpret_cast<unsigned*>(ctx->seq_gbar);
-    int grid = 1;
-    for (size_t i = 0; i < items.size(); i++) {
-        sp->layer[i] = items[i].p;
-        for (int m = 0; m < 4; m++) sp->maps[i][m] = items[i].maps[m];
-        grid = std::max(grid, std::min(items[i].p.units_total, ctx->num_sms));
-    }
-    if (getenv("RTEN_B200_VERBOSE")) fprintf(stderr, "[umma_seq] %d layers in one kernel, grid %d, class %d\n", sp->n, grid, cls);
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = 227 * 1024;  // one CTA per SM by construction: every CTA of the grid is resident (grid barrier)
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[2];
-    fill_launch_attrs(cfg, attr, false);
-    auto launch = [&](auto kern) -> cudaError_t {
-        cudaError_t e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e2 != cudaSuccess) return e2;
-        return cudaLaunchKernelEx(&cfg, kern, *sp);
-    };
-    cudaError_t e;
-    switch (cls) {
-        case 0: e = launch(umma_seq_kernel<0, 0>); break;
-        case 1: e = launch(umma_seq_kernel<0, 1>); break;
-        case 3: e = launch(umma_seq_kernel<1, 0>); break;
-        default: e = launch(umma_seq_kernel<1, 1>); break;
-    }
-    if (e != cudaSuccess) return fail_cuda(ctx, e, "umma_seq launch");
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return fail_cuda(ctx, e, "umma_seq launch");
-    count_launch(ctx);
-    return RTEN_OK;
-}
-
 // `ws`: split-K workspace of at least splitk_ws_bytes() (null: taken from the op's temporaries)
-static rten_status launch_plan(rten_ctx* ctx, const GemmLaunch& L, const Prepared& q, const Plan& pl, bool verbose,
-                               void* ws = nullptr, bool no_defer = false) {
+static rten_status launch_plan(rten_ctx* ctx, const GemmLaunch& L, const Prepared& q, const Plan& pl, bool verbose, void* ws = nullptr) {
     PlanShape ps;
     if (!plan_shape(q, pl, ps)) return RTEN_ERR_UNSUPPORTED_VALUE;
     KParams p = q.p;
@@ -610,38 +525,23 @@ static rten_status launch_plan(rten_ctx* ctx, const GemmLaunch& L, const Prepare
                 (!ee.scale || ee.scale_len == 1 || (ee.scale_len == L.N && (reinterpret_cast<uintptr_t>(ee.scale) & 15) == 0));
     // the generic epilogue takes a TMA-staged residual only on its register path (f32, act <= Relu)
     if (!fastk && (L.kind == 1 || ee.act > 1)) p.res_tma = 0;
-    PendingLaunch pend;
+    LaunchArgs args;
     if (L.kind == 0)
-        pend.plain = fastk && ee.alpha == 1.0f && ee.act <= 3 && !ee.range && (ee.r == nullptr || (p.res_tma && ee.r_scale == 1.0f));
+        args.plain = fastk && ee.alpha == 1.0f && ee.act <= 3 && !ee.range && (ee.r == nullptr || (p.res_tma && ee.r_scale == 1.0f));
     else  // integer kind: the *ToFloat operators with a scalar (or no) activation zero point and symmetric weights
-        pend.plain = fastk && ee.scale && !ee.za && !ee.zb && (ee.scale_len == 1 || ee.scale_len == L.N) && ee.act <= 3 && p.splitk == 1 &&
+        args.plain = fastk && ee.scale && !ee.za && !ee.zb && (ee.scale_len == 1 || ee.scale_len == L.N) && ee.act <= 3 && p.splitk == 1 &&
                      (ee.r == nullptr || p.res_tma) && (!ee.za8 || ee.colsum);
-    if (getenv("RTEN_B200_NO_PLAIN")) pend.plain = false;
-    pend.p = p;
-    pend.maps[0] = map_a;
-    pend.maps[1] = map_b;
-    pend.maps[2] = map_d;
-    pend.maps[3] = map_r;
-    pend.maps[4] = map_a2;
-    pend.smem_bytes = smem_bytes;
+    if (getenv("RTEN_B200_NO_PLAIN")) args.plain = false;
+    args.p = p;
+    args.maps[0] = map_a;
+    args.maps[1] = map_b;
+    args.maps[2] = map_d;
+    args.maps[3] = map_r;
+    args.maps[4] = map_a2;
+    args.smem_bytes = smem_bytes;
     // kernel class = data kind x epilogue variant (0 generic, 1 specialised, 2 specialised + out-of-line Gelu)
     const int cls = L.kind * 3 + (fastk ? (ee.act > 1 ? 2 : 1) : 0);
-    // Opt-in (RTEN_B200_SEQ=1): inside graph capture consecutive launches are collected and run as ONE sequence kernel
-    // (umma_seq_kernel).  Measured on B200 (tools/boundary_probe.py): a layer boundary inside the sequence kernel costs
-    // ~2.3 us MORE than a programmatic-dependent-launch kernel boundary (drain + grid barrier + cold operand pipe are not
-    // cheaper than what PDL already overlaps), so separate launches stay the default.
-    const char* seq_env = getenv("RTEN_B200_SEQ");
-    const bool seq_on = seq_env && atoi(seq_env) != 0;
-    if (seq_on && ctx->capturing && !p.cta2 && !p.x3_cb && !ctx->trace && !no_defer && cls % 3 != 2) {
-        auto* q2 = pending_of(ctx);
-        if (!q2->empty() && ctx->seq_class != cls) RTB_TRY(seq_flush(ctx));
-        ctx->seq_class = cls;
-        q2->push_back(pend);
-        if ((int)q2->size() == SEQ_MAX) RTB_TRY(seq_flush(ctx));
-        return RTEN_OK;
-    }
-    RTB_TRY(seq_flush(ctx));
-    return launch_single(ctx, cls, pend);
+    return launch_single(ctx, cls, args);
 }
 
 // Problem signature for the autotune cache: everything that changes which plan is fastest.

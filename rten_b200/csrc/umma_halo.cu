@@ -469,12 +469,9 @@ rten_status launch_umma_halo_conv(rten_ctx* ctx, const GemmLaunch& L, int force_
     cfg.gridDim = dim3(std::min(p.units_total, num_sms));
     cfg.blockDim = dim3(HALO_THREADS);
     cfg.dynamicSmemBytes = smem;
-    cfg.stream = launch_stream(ctx);
+    cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = getenv("RTEN_B200_NO_PDL") ? 0 : 1;
+    fill_launch_attrs(cfg, attr, false);
     cudaError_t ce = cudaFuncSetAttribute(umma_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (ce == cudaSuccess) ce = cudaLaunchKernelEx(&cfg, umma_halo_kernel, map_a, map_b, p);
     if (ce != cudaSuccess) return fail_cuda(ctx, ce, "umma_halo launch");

@@ -1,7 +1,6 @@
 // Device side of the tcgen05 GEMM / implicit-GEMM convolution: tile decode, the warp-specialised persistent kernel
-// (TMA producer / MMA issuer / TMEM allocator / two epilogue groups) and the opt-in sequence kernel.  Included ONLY by
-// umma_gemm.cu, which holds the host side (launch plans, cost model, autotuner, tensor maps).  See umma_gemm.cu's header
-// comment for the design.
+// (TMA producer / MMA issuer / TMEM allocator / two epilogue groups).  Included ONLY by umma_gemm.cu, which holds the
+// host side (launch plans, cost model, autotuner, tensor maps).  See umma_gemm.cu's header comment for the design.
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -235,9 +234,9 @@ __device__ __forceinline__ void splitk_sum(const KParams& p, int t, int sub, int
     }
 }
 
-// Per-thread pipeline state that survives from one layer of a sequence kernel to the next: parity bits of the operand
-// ring (bit s = uses of stage s so far, mod 2), of the two accumulator barriers, of the residual barriers, and the
-// running tile count that picks the accumulator stage.  Each role keeps its own copy.
+// Per-thread pipeline state of one launch: parity bits of the operand ring (bit s = uses of stage s so far, mod 2), of
+// the two accumulator barriers, of the residual barriers, and the running tile count that picks the accumulator stage.
+// Each role keeps its own copy.
 struct PipeState {
     uint32_t ring = 0, acc = 0, rphase = 0;
     int it = 0;
@@ -264,7 +263,8 @@ namespace rtb {
 template <int KIND, int FAST, int CTA2>
 __device__ __forceinline__ void run_layer(const KParams& p, const CUtensorMap* tma_a, const CUtensorMap* tma_a2,
                                           const CUtensorMap* tma_b, const CUtensorMap* tma_d, const CUtensorMap* tma_r, const SmemLayout& L,
-                                          uint32_t tmem_base, int cta_rank, int worker, int n_workers, PipeState& st) {
+                                          uint32_t tmem_base, int cta_rank, int worker, int n_workers) {
+    PipeState st;
     uint8_t* smem = L.smem;
     uint8_t* stg_base = smem + (size_t)p.stages * p.stage_bytes;
     const int nbuf = p.nbuf;
@@ -444,8 +444,7 @@ __device__ __forceinline__ void run_layer(const KParams& p, const CUtensorMap* t
 
 }
 
-// Shared-memory carve-up: a fixed 1 KB block of mbarriers first (so that it does not move when the stage geometry changes
-// from layer to layer of a sequence kernel), operand stages behind it.
+// Shared-memory carve-up: a fixed 1 KB block of mbarriers first, operand stages behind it.
 template <int KIND>
 __device__ __forceinline__ SmemLayout carve_smem(uint8_t* smem_raw) {
     // 1024-B alignment required by the 128B swizzle atoms / UMMA descriptors (base_offset = 0).
@@ -553,87 +552,10 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     if (threadIdx.x >= 32) asm volatile("griddepcontrol.wait;" ::: "memory");  // (the producer warp waits after its tile decode)
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     if (p.trace && blockIdx.x == 0 && threadIdx.x == 0) p.trace[6144 + 1102] = clock64();  // predecessor complete
-    PipeState st;
-    run_layer<KIND, FAST, CTA2>(p, &tma_a, &tma_a2, &tma_b, &tma_d, &tma_r, L, tmem_base, cta_rank, worker, n_workers, st);
+    run_layer<KIND, FAST, CTA2>(p, &tma_a, &tma_a2, &tma_b, &tma_d, &tma_r, L, tmem_base, cta_rank, worker, n_workers);
     if (p.trace && blockIdx.x == 0 && threadIdx.x == 0) p.trace[6144 + 1103] = clock64();  // control thread done
     kernel_teardown<CTA2>(tmem_base);
     if (p.trace && blockIdx.x == 0 && threadIdx.x == 0) p.trace[6144 + 1104] = clock64();  // exit
-}
-
-// ------------------------------------------------------------------------------------------
-// Sequence kernel: up to SEQ_MAX consecutive launches (layers of a captured op list) run inside ONE persistent
-// kernel.  Between two layers every CTA drains its output stores and meets the others at a grid-wide barrier (an
-// arrival counter in global memory): a layer boundary costs one barrier round trip plus one TMA latency instead of a
-// kernel launch, TMEM allocation, tensor-map fetch and a cold pipeline.  Layer parameters and tensor maps live in the
-// kernel parameter block (constant bank), indexed by the layer number.
-// ------------------------------------------------------------------------------------------
-constexpr int SEQ_MAX = 28;
-struct SeqParams {
-    int n;
-    int pad;
-    unsigned* gbar;  // arrival counter, zero between launches
-    CUtensorMap maps[SEQ_MAX][4];
-    KParams layer[SEQ_MAX];
-};
-static_assert(sizeof(SeqParams) <= 32764, "kernel parameter block too large");
-
-__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-template <int KIND, int FAST>
-__global__ void __launch_bounds__(NUM_THREADS, 1) umma_seq_kernel(const __grid_constant__ SeqParams sp) {
-    extern __shared__ uint8_t smem_raw[];
-    const SmemLayout L = carve_smem<KIND>(smem_raw);
-    if (threadIdx.x == 0) {
-        tma_prefetch_desc(&sp.maps[0][0]);
-        tma_prefetch_desc(&sp.maps[0][1]);
-    }
-    const uint32_t tmem_base = kernel_setup<0>(L);
-    if (threadIdx.x >= 32) asm volatile("griddepcontrol.wait;" ::: "memory");
-    PipeState st;
-    const int warp = threadIdx.x >> 5;
-    for (int l = 0; l < sp.n; l++) {
-        const KParams& p = sp.layer[l];
-        if (l + 1 == sp.n) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        run_layer<KIND, FAST, 0>(p, &sp.maps[l][0], &sp.maps[l][0], &sp.maps[l][1], &sp.maps[l][2], &sp.maps[l][3], L, tmem_base, 0,
-                                 (int)blockIdx.x, (int)gridDim.x, st);
-        if (l + 1 < sp.n) {
-            // ---- layer boundary: this CTA's outputs are complete and visible, then wait for every other CTA's
-            if (warp >= 4) {
-                asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // TMA stores performed (issuer threads)
-                asm volatile("fence.proxy.async;" ::: "memory");
-                __threadfence();
-            }
-            if (threadIdx.x == 32) {  // idle until the barrier anyway: fetch the next layer's tensor maps
-                tma_prefetch_desc(&sp.maps[l + 1][0]);
-                tma_prefetch_desc(&sp.maps[l + 1][1]);
-                tma_prefetch_desc(&sp.maps[l + 1][2]);
-            }
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                __threadfence();
-                atomicAdd(sp.gbar, 1u);
-                const unsigned target = gridDim.x * (unsigned)(l + 1);
-                uint32_t spins = 0;
-                while (ld_acquire_gpu(sp.gbar) < target) {
-                    __nanosleep(32);
-                    if (++spins > (1u << 25)) __trap();  // > ~1 s: a CTA of the grid never arrived
-                }
-                __threadfence();
-            }
-            __syncthreads();
-            asm volatile("fence.proxy.async;" ::: "memory");
-        }
-    }
-    // re-arm the arrival counter: the last CTA to leave (everyone has passed every barrier by then) zeroes it
-    if (threadIdx.x == 0) {
-        const unsigned old = atomicAdd(sp.gbar, 1u);
-        if (old == gridDim.x * (unsigned)sp.n - 1u) *reinterpret_cast<volatile unsigned*>(sp.gbar) = 0u;
-    }
-    kernel_teardown<0>(tmem_base);
 }
 
 }  // namespace rtb

@@ -434,20 +434,10 @@ def check_plans(rt, oracle):
 
 
 # ------------------------------------------------------------------------------------------
-def check_sequence(rt, oracle):
-    """Inside graph capture consecutive tensor-core launches are fused into persistent sequence kernels (grid barrier
-    between layers).  Replaying the graph must reproduce the eager results bit for bit (same plans, same arithmetic),
-    for chains shorter and longer than one kernel's layer capacity, with residual links, and more than once.
-    (The sequence kernel is opt-in through RTEN_B200_SEQ=1, set here for the duration of the check.)"""
-    import os
-    os.environ["RTEN_B200_SEQ"] = "1"
-    try:
-        return _check_sequence(rt, oracle)
-    finally:
-        os.environ.pop("RTEN_B200_SEQ", None)
-
-
-def _check_sequence(rt, oracle):
+def check_graph_replay(rt, oracle):
+    """A captured graph of consecutive tensor-core launches must reproduce the eager results bit for bit (same plans,
+    same arithmetic) when replayed: for an 8-layer and a 45-layer conv chain with residual links, more than once, and
+    for independent integer launches in one capture."""
     ctx = new_ctx(rt)
     r = oracle.XorShiftRng(321)
 
@@ -460,7 +450,7 @@ def _check_sequence(rt, oracle):
     # a: bottleneck-like chain with residual links (index of the producing layer, -1 = the input)
     chain_a = [conv_layer(64, 128, 1), conv_layer(128, 128, 3), conv_layer(128, 128, 1, res=0), conv_layer(128, 64, 3),
                conv_layer(64, 256, 1), conv_layer(256, 64, 1), conv_layer(64, 64, 3, res=5), conv_layer(64, 512, 1, act=0)]
-    # b: longer than SEQ_MAX layers -> split over several sequence kernels
+    # b: a 45-layer chain
     chain_b = [conv_layer(64, 64, 1, res=(i - 2 if i >= 2 and i % 3 == 0 else None)) for i in range(45)]
     x = ctx.to_device(r.uniform((4, 64, 28, 28)), channels_last=True)
 
@@ -489,9 +479,9 @@ def _check_sequence(rt, oracle):
             g.launch()
             ctx.sync()
             for i, (t, w) in enumerate(zip(eager, want)):
-                assert_bit_exact(t.numpy(), w, f"sequence chain {name} layer {i} replay {rep}")
+                assert_bit_exact(t.numpy(), w, f"graph replay chain {name} layer {i} replay {rep}")
         worst_layers = max(worst_layers, len(chain))
-    # integer launches in one capture (independent problems, one sequence kernel)
+    # integer launches in one capture (independent problems)
     a8 = [r.u8((200, 512)) for _ in range(3)]
     b8 = [r.i8((512, 160)) for _ in range(3)]
     az, bz = r.u8((200,)), r.i8((160,))
@@ -507,7 +497,7 @@ def _check_sequence(rt, oracle):
     g.launch()
     ctx.sync()
     for o, w in zip(outs, want):
-        assert_bit_exact(o.numpy(), w, "sequence MatMulInteger")
+        assert_bit_exact(o.numpy(), w, "graph replay MatMulInteger")
     return f"chains of up to {worst_layers} layers replayed bit-exactly"
 
 
@@ -1653,7 +1643,7 @@ ALL_CHECKS = [
     ("dql", check_dql), ("glue", check_glue), ("matmul_small", check_matmul_small), ("matmul_shapes", check_matmul_shapes),
     ("matmul_bert", check_matmul_bert), ("gemm_op", check_gemm_op), ("matmul_integer", check_matmul_integer),
     ("conv_basic", check_conv_basic), ("conv_stride", check_conv_stride), ("conv_more", check_conv_more),
-    ("conv_integer", check_conv_integer), ("plans", check_plans), ("tf32x3", check_tf32x3), ("sequence", check_sequence), ("conv_integer_fused", check_conv_integer_fused),
+    ("conv_integer", check_conv_integer), ("plans", check_plans), ("tf32x3", check_tf32x3), ("graph_replay", check_graph_replay), ("conv_integer_fused", check_conv_integer_fused),
     ("resnet50_int8_model", check_resnet50_int8_model), ("gpt2_int8_kvcache", check_gpt2_int8_kvcache), ("mnist_model", check_mnist_model), ("resnet50_model", check_resnet50_model), ("bert_model", check_bert_model),
     ("model_executor", check_model_executor), ("generator", check_generator), ("halo_conv", check_halo_conv), ("quantized_linear", check_quantized_linear), ("attention_decode", check_attention_decode), ("attention_encoder", check_attention_encoder), ("gelu_epilogue", check_gelu_epilogue), ("skinny_f32", check_skinny_f32),
     ("reference_rule_f32", check_reference_rule_f32), ("graph_pool_isolation", check_graph_pool_isolation),

@@ -1,6 +1,6 @@
 """Marginal cost of one more dependent tensor-core launch: time CUDA graphs holding 1, 2, 4, 8, 16 copies of the same
-layer (chained: copy i reads the output of copy i-1 when shapes allow, else the same input), with the sequence kernel on
-and off.  Slope = steady-state time per layer, intercept = graph launch overhead."""
+layer (chained: copy i reads the output of copy i-1 when shapes allow, else the same input), each a separate launch
+chained by programmatic dependent launch.  Slope = steady-state time per layer, intercept = graph launch overhead."""
 import os
 
 os.environ.setdefault("RTEN_B200_F32_MODE", "tf32")  # these tools measure the single-pass TF32 kernels unless told otherwise
@@ -60,17 +60,12 @@ def time_graph(ctx, run, n, reps=30):
 
 
 cases = [(64, 64, 3, 56), (128, 128, 3, 28), (256, 256, 3, 14), (512, 512, 3, 7), (64, 64, 1, 56), (256, 256, 1, 14)]
-for mode in ("single", "seq"):
-    if mode == "single":
-        os.environ.pop("RTEN_B200_SEQ", None)
-    else:
-        os.environ["RTEN_B200_SEQ"] = "1"  # opt-in persistent sequence kernel (grid barrier between layers)
-    os.environ["RTEN_B200_NO_CTA2"] = "1"
-    ctx = rt.Context(0, stream=stream.cuda_stream)
-    ctx.set_autotune(True)
-    for (ci, co, k, hw) in cases:
-        run = build(ctx, ci, co, k, hw)
-        ns = [1, 2, 4, 8, 16]
-        t = [time_graph(ctx, run, n) for n in ns]
-        slope = (t[-1] - t[2]) / (ns[-1] - ns[2])
-        print(f"{mode:6s} conv {k}x{k} {ci}->{co} @{hw}: " + " ".join(f"n={n}:{v:.1f}us" for n, v in zip(ns, t)) + f"  | marginal {slope:.2f} us/layer", flush=True)
+os.environ["RTEN_B200_NO_CTA2"] = "1"
+ctx = rt.Context(0, stream=stream.cuda_stream)
+ctx.set_autotune(True)
+for (ci, co, k, hw) in cases:
+    run = build(ctx, ci, co, k, hw)
+    ns = [1, 2, 4, 8, 16]
+    t = [time_graph(ctx, run, n) for n in ns]
+    slope = (t[-1] - t[2]) / (ns[-1] - ns[2])
+    print(f"single conv {k}x{k} {ci}->{co} @{hw}: " + " ".join(f"n={n}:{v:.1f}us" for n, v in zip(ns, t)) + f"  | marginal {slope:.2f} us/layer", flush=True)
